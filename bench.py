@@ -11,6 +11,7 @@ through the host-buffer path a user calls (loro_b200.import_batch -> lb_import_b
 timed region, JSON + status + re-exported blobs read back to the host; large batches go as two overlapping sub-batches).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2|C3|C4|C5] [--docs D] [--ops-per-doc 10000]
+                  [--dump-outputs DIR]   # what the last timed step returned, as DIR/*.npy (dump_outputs)
   python bench.py --impl reference ...     # the CPU arm: the oracle port of the reference path on host cores
 
 Under torchrun (N>1) every rank imports its own shard of documents (weak scaling: per-GPU work fixed) and
@@ -56,7 +57,15 @@ def parse_args():
     ap.add_argument("--cpu-sample-docs", type=int, default=0)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-export", action="store_true", help="skip the re-export phase (import + state only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs; "
+                         "under torchrun, rank 0's documents)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's outputs; the reference arm has none")
+    return args
 
 
 def peaks():
@@ -224,17 +233,21 @@ def workload_text(args, n_docs, extra=""):
             f"one FastUpdates blob per doc (SURVEY.md 8d){extra}")
 
 
+GEN_CORES = 16   # host cores the generation budget below is sized for
+
+
 def affordable_distinct(args, world, n_docs):
-    """How many DISTINCT documents this rank's share of the host cores can generate in about 90 s
+    """How many DISTINCT documents this rank's share of GEN_CORES host cores can generate in about 90 s
     (~1.2 M generated atom ops/s/core); the batch is filled by cycling through them (every copy has its own bytes
-    in HBM; `distinct_docs_per_gpu` in the config says how many there are)."""
+    in HBM; `distinct_docs_per_gpu` in the config says how many there are).  The budget is fixed rather than taken
+    from this host's cores, so that the same arguments give the same inputs on every machine."""
     if args.config == "C2" and args.c2_distinct_peers:
         return n_docs
     if args.config in ("C2", "C4"):
         return 1
     if args.distinct:
         return min(args.distinct, n_docs)
-    cores = max(1, (host_cores() or 1) // max(1, world))
+    cores = max(1, GEN_CORES // max(1, world))
     if args.config == "C5":   # ~0.7 M generated tree ops/s/core
         return max(64, min(n_docs, int(cores * 0.7e6 * 90 / (args.tree_nodes + args.peers * args.tree_moves))))
     return max(64, min(n_docs, int(cores * 1.2e6 * 90 / args.ops_per_doc)))
@@ -347,6 +360,60 @@ def ncu_traffic(kernel_key, rows):
         return None
 
 
+DUMP_DOCS = 64                # documents sampled, with a fixed seed, for the per-document outputs
+DUMP_STREAM_BYTES = 6000000   # bytes kept of each per-document byte stream (JSON, re-export), shared by the sample
+
+
+def dump_outputs(b, out_dir, with_export):
+    """--dump-outputs DIR: what the timed path returned to its caller in the last timed step, as .npy files by which two
+    builds can be compared (about 50 MB at most).  64-bit values (peer ids, state_hash) are split into two float64
+    columns, high and low 32 bits, so that every value is exact.
+      counters.npy          [10, 2]  the batch counters, in loro_b200.shard.COUNTER_KEYS order
+      docs.npy              [K]      the K = min(n_docs, DUMP_DOCS) sampled documents (fixed seed, ascending)
+      status.npy            [K]      ImportStatus code of each
+      status_spans.npy      [S, 6]   sample row, 0 = success / 1 = pending, peer hi, peer lo, start, end
+      vv.npy, frontiers.npy [V, 4]   sample row, peer hi, peer lo, counter
+      json.npy              float32  each sampled document's JSON bytes, back to back, at most DUMP_STREAM_BYTES // K
+                                     of each (a prefix); json_offsets.npy [K + 1] delimits them
+      json_len.npy          [K]      the length of the whole JSON; json_sha256.npy [K, 32] its SHA-256, byte by byte
+      export*.npy                    the same four for the re-exported blob (not with --no-export)"""
+    import hashlib
+    import numpy as np
+    from loro_b200.shard import COUNTER_KEYS
+
+    def words(v):
+        return (int(v) >> 32) & 0xFFFFFFFF, int(v) & 0xFFFFFFFF
+
+    c = b.counters()
+    out = {"counters": np.array([words(c[k]) for k in COUNTER_KEYS], dtype=np.float64)}
+    k = min(b.n_docs, DUMP_DOCS)
+    docs = [int(i) for i in np.sort(np.random.default_rng(0).choice(b.n_docs, size=k, replace=False))]
+    out["docs"] = np.array(docs, dtype=np.float64)
+    status, spans, vv, fr = [], [], [], []
+    for r, i in enumerate(docs):
+        st = b.status(i)
+        status.append(st.code)
+        for kind, d in ((0, st.success), (1, st.pending or {})):
+            spans += [(r, kind, *words(p), s, e) for p, (s, e) in sorted(d.items())]
+        vv += [(r, *words(p), n) for p, n in sorted(b.oplog_vv(i).items())]
+        fr += [(r, *words(p), n) for p, n in b.oplog_frontiers(i)]
+    out["status"] = np.array(status, dtype=np.float64)
+    out["status_spans"] = np.array(spans, dtype=np.float64).reshape(-1, 6)
+    out["vv"] = np.array(vv, dtype=np.float64).reshape(-1, 4)
+    out["frontiers"] = np.array(fr, dtype=np.float64).reshape(-1, 4)
+    cap = DUMP_STREAM_BYTES // k
+    for name, get in [("json", b.json_bytes)] + ([("export", b.export_updates)] if with_export else []):
+        whole = [get(i) for i in docs]
+        kept = [w[:cap] for w in whole]
+        out[name] = np.frombuffer(b"".join(kept), dtype=np.uint8).astype(np.float32)
+        out[name + "_offsets"] = np.cumsum([0] + [len(x) for x in kept]).astype(np.float64)
+        out[name + "_len"] = np.array([len(w) for w in whole], dtype=np.float64)
+        out[name + "_sha256"] = np.array([list(hashlib.sha256(w).digest()) for w in whole], dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     args = parse_args()
     if args.impl == "reference":
@@ -388,20 +455,22 @@ def main():
 
     xflags = 0 if args.no_export else loro_b200.api.LB_FLAG_EXPORT
 
-    def step():
+    def step(keep=False):
         b = loro_b200.import_batch_device(d_bytes.data_ptr(), offs, lens, device=local, flags=xflags, keep=d_bytes)
         c = b.counters()
         if world > 1:
             gather_counters(c, device=dev)  # the one collective of the path: per-shard summary counters (NCCL)
         tm = b.timings()
+        if keep:
+            return c, tm, b
         b.close()
-        return c, tm
+        return c, tm, None
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     for _ in range(args.warmup):
-        c, tm = step()
+        c, tm, _ = step()
     assert c["docs_ok"] == n_docs, c
     atoms_per_step = c["atom_ops"]
     if world > 1:
@@ -414,8 +483,9 @@ def main():
     t_wall = time.time()
     phase = {}
     launches = 0
-    for _ in range(args.steps):
-        c, tm = step()
+    for s in range(args.steps):
+        # rank 0 keeps the last step's batch open for --dump-outputs (closed below, once the timed region has ended)
+        c, tm, last = step(keep=bool(args.dump_outputs) and rank == 0 and s == args.steps - 1)
         launches += tm["kernel_launches"]
         for k in ("frame", "decode", "resolve", "classify", "integrate", "tree", "materialise", "reexport", "total_device",
                   "alloc_host_ms", "host_call_ms", "host_tail_ms"):
@@ -431,6 +501,9 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dev_ms = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
+    if last is not None:
+        dump_outputs(last, args.dump_outputs, with_export=bool(xflags))
+        last.close()
     total_atoms = atoms_per_step * world
     value = total_atoms * args.steps / (dev_ms * 1e-3)
     ms_per_step = dev_ms / args.steps

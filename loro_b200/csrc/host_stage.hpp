@@ -17,6 +17,11 @@
 #include <vector>
 
 namespace lbstage {
+// Internal linkage: the statics of inline functions below (rings, caches, worker pool) would otherwise be GNU-unique
+// symbols, which the dynamic loader shares between every library of the process that defines them -- a second build
+// of the engine loaded next to this one (the emulated test build, a tuning variant) would hand this one its pinned
+// slots and CUDA events.
+namespace {
 
 constexpr size_t SLOT_BYTES = 32u << 20;
 constexpr int N_SLOTS = 4;
@@ -242,4 +247,5 @@ inline bool download(const uint8_t* d_src, uint8_t* dst, size_t total, cudaStrea
     return true;
 }
 
+}  // namespace
 }  // namespace lbstage

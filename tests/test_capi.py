@@ -38,10 +38,26 @@ def test_no_cpu_fallback_without_a_device():
 
 
 def test_sass_is_sm100a(lib):
+    import shutil
     import subprocess
     import loro_b200
-    out = subprocess.run(["cuobjdump", "-lelf", loro_b200.library_path()], capture_output=True, text=True).stdout
+    # the toolkit that build() compiles with, also when its bin/ is not on PATH
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(nvcc), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", loro_b200.library_path()], capture_output=True, text=True).stdout
     assert "sm_100a" in out, out
+
+
+def test_library_shares_no_state_with_other_builds_in_the_process(lib):
+    """The library defines no GNU-unique symbol of its own: the dynamic loader binds such a symbol to the first library
+    of the process that defines it, so a second build of the engine (the emulated one, loaded first when this suite runs
+    in one process) would hand the CUDA library its host staging ring."""
+    import subprocess
+    import loro_b200
+    out = subprocess.run(["nm", "-DC", "--defined-only", loro_b200.library_path()], capture_output=True, text=True,
+                         check=True).stdout
+    unique = [ln for ln in out.splitlines() if ln.split()[1:2] == ["u"] and " std::" not in ln]
+    assert not unique, unique
 
 
 def test_plain_c_caller_compiles_links_and_fails_loudly_without_a_device(lib, tmp_path):

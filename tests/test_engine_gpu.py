@@ -470,6 +470,27 @@ def test_config_c4_full_size_against_committed_oracle_digests(golden_dir, which)
     assert len(ex) == want["export_len"] and xxh(ex) == want["export_xxh32"]
 
 
+def test_library_next_to_the_emulated_build():
+    """The emulated test build and the CUDA library in one process, the emulated one used first (as when the whole suite
+    runs in one pytest process): each keeps its own host staging rings, and both give the same document."""
+    import subprocess
+    import sys
+    emu = os.path.join(HERE, "emu", "libloro_b200_emu.so")
+    subprocess.check_call([os.path.join(HERE, "emu", "build_emu.sh")])
+    code = (
+        "import sys; sys.path.insert(0, %r)\n"
+        "import loro_b200\n"
+        "from tests import workloads\n"
+        "blob = workloads.make_doc_history(5, n_sites=2, n_ops=60)[0]\n"
+        "a = loro_b200.import_batch([blob], lib_path=%r)\n"
+        "b = loro_b200.import_batch([blob])\n"
+        "assert b.status(0).code == 0 and a.json_bytes(0) == b.json_bytes(0)\n"
+        "print('ok')\n"
+    ) % (os.path.dirname(HERE), emu)
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0 and out.stdout.strip() == "ok", out.stderr[-2000:]
+
+
 def test_plain_c_caller_runs_against_the_library(tmp_path, golden_dir):
     """examples/c/import_and_docset.c (plain C99 against include/loro_b200.h): import_batch of two updates of one document,
     then the same updates one call at a time into a docset document"""
